@@ -2,6 +2,7 @@
 """bench.py — driver contract for the B200-native DWA hot path.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cycle|sweep]
+                    [--dump-outputs DIR]
 
 A "step" is one DWA control cycle of one robot on BASELINE.json configs[1]: differential drive,
 9 900 velocity slots x 50 points (dt 0.02 s, 1 s horizon) against a 100 000-point synthetic cloud,
@@ -25,6 +26,13 @@ config.distribution = the worst one, and e2e.by_distribution carries p50/p90/p99
          run; `--workload sweep` makes that sweep the headline (value, "scaling": "strong").
   --impl reference   the CPU restatement of the reference path (oracle/, or oracle/_ref when the
          reference's own sources were compiled) with all host threads on the same config.
+  --dump-outputs DIR   after the timed steps, rank 0 writes what the headline's timed path returned in
+         its last step. Cycle: the winner record of the LAST timed cycle as the public call returns it,
+         DIR/winner.npy (float64: found, cost, slot, n_admissible, n_slots, n_points) and
+         DIR/trajectory_{vx,vy,omega,x,y}.npy (float32 rows of the winning trajectory). Sweep
+         (--workload sweep): DIR/sweep_winners.npy, float64 [robots, 4] = found, cost, slot,
+         n_admissible of every robot in the last timed replay, gathered in robot order. The clouds are
+         seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -286,6 +294,25 @@ def pct(a, q):
     return float(np.percentile(a, q) * 1e3)
 
 
+def dump_cycle_outputs(out_dir, r):
+    """--dump-outputs: the winner record `r` (TrajSearchResult) of one cycle, as a caller receives it."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {
+        "winner": np.array([r.is_found, r.cost, r.slot, r.n_admissible, r.n_slots, r.n_points], np.float64),
+        "trajectory_vx": np.asarray(r.vx, np.float32), "trajectory_vy": np.asarray(r.vy, np.float32),
+        "trajectory_omega": np.asarray(r.omega, np.float32),
+        "trajectory_x": np.asarray(r.x, np.float32), "trajectory_y": np.asarray(r.y, np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_sweep_outputs(out_dir, rows):
+    """--dump-outputs, --workload sweep: one (found, cost, slot, n_admissible) row per robot."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "sweep_winners.npy"), np.array(rows, np.float64).reshape(-1, 4))
+
+
 # =================================================================================================
 # CPU legs (the only places that touch oracle/): --impl reference and the cpu_baseline subprocess
 # =================================================================================================
@@ -543,7 +570,7 @@ def measure_distribution(pkg, planner, wl, name, rank, seg, vel, pose, n_lat, re
     return rec, clouds, lat, wall
 
 
-def run_sweep(pkg, wl, kw, path, seg, world, rank, local, dist, robots_total, iters):
+def run_sweep(pkg, wl, kw, path, seg, world, rank, local, dist, robots_total, iters, dump_dir=None):
     """north_star config 5: `robots_total` independent robots (own cloud seed, own current velocity),
     sharded contiguously by robot id across the ranks; no data-path collective, the final gather
     carries 20 bytes per robot. Returns a dict for the JSON line (rank 0) or None."""
@@ -580,6 +607,10 @@ def run_sweep(pkg, wl, kw, path, seg, world, rank, local, dist, robots_total, it
     barrier(dist, local)
     ms = max_over_ranks(dist, ms, local)
     assert [x[2] for x in res] == [x[2] for x in res2], "replayed sweep changed its winners"
+    if dump_dir:
+        last = gather_results(dist, res2, world, rank)
+        if rank == 0:
+            dump_sweep_outputs(dump_dir, last)
     P = planner.num_points
     units = sum_over_ranks(dist, float(sum(slots)) * P, local)
     gathered = gather_results(dist, res, world, rank)
@@ -754,6 +785,8 @@ def run_ours(args):
     n_slots, P = last.n_slots, last.n_points
     units_per_step = n_slots * P
     value = world * steps * units_per_step / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0 and args.workload == "cycle":
+        dump_cycle_outputs(args.dump_outputs, last)
 
     # ---- dominant kernels (rollout+collision+cost) timed live with CUDA events -------------------
     ksteps = min(max(steps, 100), 500)
@@ -792,7 +825,8 @@ def run_ours(args):
 
     sweep = None
     if args.sweep_robots > 0:
-        sweep = run_sweep(pkg, wl, kw, path, seg, world, rank, local, dist, args.sweep_robots, args.sweep_iters)
+        sweep = run_sweep(pkg, wl, kw, path, seg, world, rank, local, dist, args.sweep_robots, args.sweep_iters,
+                          args.dump_outputs if args.workload == "sweep" else None)
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()
@@ -947,7 +981,13 @@ def main():
     ap.add_argument("--sweep-robots", type=int, default=SWEEP_ROBOTS,
                     help="robots of the batched multi-robot sweep (config 5), 0 = skip")
     ap.add_argument("--sweep-iters", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.dump_outputs and args.workload == "sweep" and args.sweep_robots <= 0:
+        ap.error("--dump-outputs with --workload sweep needs --sweep-robots > 0")
     claim_stdout()
     if args.cpu_baseline_only:
         return run_cpu_baseline_only(args)
