@@ -399,6 +399,51 @@ int32_t kc_planner_batch_replay(kc_planner *p, int32_t n_iters, float *total_ms,
                                 kc_batch_result *results);
 
 /* =============================================================================================
+ * Multi-robot DWA controller: R robots, each with its own reference path, state, control limits
+ * and sensor data, stepped together in one batched launch set per chunk of robots. For every robot
+ * r a step returns exactly what a kc_dwa handle with the same configuration, path, state and
+ * sensor data returns from kc_dwa_compute_*: found, slot, cost bits, n_admissible, n_slots, P, the
+ * winner rows, every kc_dwa_info field, the clamped command and the goal flag. The latest command
+ * is kept when no trajectory is found. Custom cost callbacks and the debug velocity search stay
+ * with kc_dwa.
+ * Sensor data uses the layout of kc_planner_batch_cloud: robot r's cloud is xyz + 3*offsets[r]
+ * (counts[r] points), its scan ranges + offsets[r] / angles + offsets[r] (counts[r] beams); robots
+ * may share slices; page-locked clouds are DMA-ed directly. A step takes one sensor kind.
+ * ========================================================================================== */
+typedef struct kc_fleet kc_fleet;
+typedef struct kc_fleet_result {
+  int32_t found;
+  float cost;
+  int32_t slot, n_points, n_slots, n_admissible;
+  double cmd[3]; /* command after this step, exactly what kc_dwa_get_command would return */
+} kc_fleet_result;
+/* follower: NULL = defaults. Fails with KC_ERR_CUDA without a device. */
+int32_t kc_fleet_create(const kc_planner_config *cfg, const kc_follower_params *follower, int32_t n_robots,
+                        kc_fleet **out);
+void kc_fleet_destroy(kc_fleet *f);
+/* the shared planner: weights, resolution, max range, drop mode, tuning keys */
+kc_planner *kc_fleet_planner(kc_fleet *f);
+/* Follower::setCurrentPath of one robot; its interpolated path goes to the device once, here */
+int32_t kc_fleet_set_current_path(kc_fleet *f, int32_t robot, const float *x, const float *y, int32_t n,
+                                  int32_t interpolate);
+int32_t kc_fleet_clear_current_path(kc_fleet *f, int32_t robot);
+/* states: [R x 4] doubles (x, y, yaw, speed) */
+int32_t kc_fleet_set_current_states(kc_fleet *f, const double *states);
+/* Controller limits of every robot (as kc_dwa_set_control_limits) */
+int32_t kc_fleet_set_control_limits(kc_fleet *f, double vx_max, double vy_max, double omega_max);
+/* one step of every robot. vel: [R x 3]; results: [R]; info: [R] or NULL. A robot without a path
+ * fails the call with KC_ERR_INVALID_ARG naming it. */
+int32_t kc_fleet_compute_cloud(kc_fleet *f, const double *vel, const float *xyz, const int64_t *offsets,
+                               const int32_t *counts, kc_fleet_result *results, kc_dwa_info *info);
+int32_t kc_fleet_compute_scan(kc_fleet *f, const double *vel, const double *ranges, const double *angles,
+                              const int64_t *offsets, const int32_t *counts, kc_fleet_result *results,
+                              kc_dwa_info *info);
+/* the winner record of one robot's last step (rows valid until the next call on the fleet) */
+int32_t kc_fleet_get_trajectory(const kc_fleet *f, int32_t robot, kc_cycle_result *out);
+/* Follower::isGoalReached of every robot: reached [R] */
+int32_t kc_fleet_is_goal_reached(kc_fleet *f, int32_t *reached);
+
+/* =============================================================================================
  * Local mapper. ref: include/mapping/local_mapper_gpu.h:12-147 (LocalMapperGPU ctor + 2
  * scanToGrid overloads); arithmetic follows the reference CPU LocalMapper::scanToGrid
  * (src/mapping/local_mapper.cpp:127-159,204-251), which is the parity target.

@@ -168,6 +168,9 @@ ABI_SYMBOLS = [
     "kc_pointcloud_to_laserscan", "kc_pointcloud_to_laserscan_step", "kc_mapper_cloud_to_grid_bayesian",
     "kc_critical_zone_create", "kc_critical_zone_destroy", "kc_critical_zone_check_scan",
     "kc_critical_zone_check_cloud", "kc_critical_zone_replay",
+    "kc_fleet_create", "kc_fleet_destroy", "kc_fleet_planner", "kc_fleet_set_current_path",
+    "kc_fleet_clear_current_path", "kc_fleet_set_current_states", "kc_fleet_set_control_limits",
+    "kc_fleet_compute_cloud", "kc_fleet_compute_scan", "kc_fleet_get_trajectory", "kc_fleet_is_goal_reached",
 ]
 
 _lib = None
@@ -192,6 +195,9 @@ def lib():
         L.kc_collision_destroy.argtypes = [C.c_void_p]
         L.kc_collision_get_radius.restype = C.c_float
         L.kc_collision_get_radius.argtypes = [C.c_void_p]
+        L.kc_fleet_destroy.argtypes = [C.c_void_p]
+        L.kc_fleet_planner.restype = C.c_void_p
+        L.kc_fleet_planner.argtypes = [C.c_void_p]
         L.kc_debug_atan2f.restype = C.c_float
         L.kc_debug_atan2f.argtypes = [C.c_float, C.c_float]
         _lib = L
@@ -756,6 +762,181 @@ class DWA:
         slots = np.ctypeslib.as_array(s.slots, shape=(n,)).copy() if n else np.zeros(0, np.int32)
         return dict(vx=_rows(s.vx, n, P - 1), vy=_rows(s.vy, n, P - 1), omega=_rows(s.omega, n, P - 1),
                     x=_rows(s.x, n, P), y=_rows(s.y, n, P), slots=slots, P=P)
+
+
+class FleetResult(C.Structure):  # kc_fleet_result
+    _fields_ = [("found", C.c_int32), ("cost", C.c_float), ("slot", C.c_int32), ("n_points", C.c_int32),
+                ("n_slots", C.c_int32), ("n_admissible", C.c_int32), ("cmd", C.c_double * 3)]
+
+
+def _fleet_rows(a, R, k, name):
+    """[R x k] float64, C-contiguous; ValueError on any other shape."""
+    a = np.asarray(a, dtype=np.float64)
+    if a.shape != (R, k):
+        raise ValueError(f"{name} must have shape ({R}, {k}), got {a.shape}")
+    return np.ascontiguousarray(a)
+
+
+def _fleet_extents(R, offsets, counts):
+    offsets, counts = np.asarray(offsets), np.asarray(counts)
+    if offsets.shape != (R,) or counts.shape != (R,):
+        raise ValueError(f"offsets and counts must have shape ({R},), got {offsets.shape} and {counts.shape}")
+    if (offsets < 0).any() or (counts < 0).any():
+        raise ValueError("offsets and counts must be non-negative")
+    return np.ascontiguousarray(offsets, np.int64), np.ascontiguousarray(counts, np.int32)
+
+
+def fleet_pack_clouds(R, clouds):
+    """clouds: a list of R [n_r x 3] arrays, or the flat form (xyz, offsets, counts) of
+    Planner.batch_cloud (a PinnedArray's .array is DMA-ed without a staging copy).
+    Returns (xyz [n x 3] float32, offsets int64 [R], counts int32 [R])."""
+    if isinstance(clouds, tuple):
+        if len(clouds) != 3:
+            raise ValueError("flat clouds are (xyz, offsets, counts)")
+        xyz = _f32(clouds[0])
+        if xyz.size % 3:
+            raise ValueError("cloud must hold xyz triples")
+        xyz = xyz.reshape(-1, 3)
+        offsets, counts = _fleet_extents(R, clouds[1], clouds[2])
+        if R and int((offsets + counts).max()) > len(xyz):
+            raise ValueError("offsets + counts exceed the cloud")
+        return xyz, offsets, counts
+    if len(clouds) != R:
+        raise ValueError(f"expected {R} clouds, got {len(clouds)}")
+    parts = []
+    for c in clouds:
+        c = np.asarray(c, np.float32)
+        if c.size % 3:
+            raise ValueError("cloud must hold xyz triples")
+        parts.append(c.reshape(-1, 3))
+    counts = np.array([len(c) for c in parts], np.int32)
+    offsets = np.zeros(R, np.int64)
+    offsets[1:] = np.cumsum(counts[:-1])
+    xyz = _f32(np.concatenate(parts, axis=0)) if R else np.zeros((0, 3), np.float32)
+    return xyz, offsets, counts
+
+
+def fleet_pack_scans(R, scans):
+    """scans: a list of R (ranges, angles) pairs, or the flat form (ranges, angles, offsets, counts).
+    Returns (ranges float64, angles float64, offsets int64 [R], counts int32 [R])."""
+    if isinstance(scans, tuple):
+        if len(scans) != 4:
+            raise ValueError("flat scans are (ranges, angles, offsets, counts)")
+        r, a = _f64(scans[0]).ravel(), _f64(scans[1]).ravel()
+        if len(r) != len(a):
+            raise ValueError("LaserScan ranges and angles must have the same size")
+        offsets, counts = _fleet_extents(R, scans[2], scans[3])
+        if R and int((offsets + counts).max()) > len(r):
+            raise ValueError("offsets + counts exceed the scan arrays")
+        return r, a, offsets, counts
+    if len(scans) != R:
+        raise ValueError(f"expected {R} scans, got {len(scans)}")
+    rs, angs = [], []
+    for sc in scans:
+        r, a = np.asarray(sc[0], np.float64).ravel(), np.asarray(sc[1], np.float64).ravel()
+        if len(r) != len(a):
+            raise ValueError("LaserScan ranges and angles must have the same size")
+        rs.append(r)
+        angs.append(a)
+    counts = np.array([len(r) for r in rs], np.int32)
+    offsets = np.zeros(R, np.int64)
+    offsets[1:] = np.cumsum(counts[:-1])
+    return _f64(np.concatenate(rs)), _f64(np.concatenate(angs)), offsets, counts
+
+
+class DWAFleet:
+    """R DWA controllers stepped together (include/kompass_b200.h, kc_fleet_*). Each robot has its
+    own path, state and sensor data; a step returns for every robot what a DWA handle with the same
+    configuration and inputs returns, from one batched launch set per chunk of robots. All robots
+    share the configuration, the control limits and the planner settings (`planner`)."""
+
+    def __init__(self, cfg, follower=None, n_robots=1):
+        n_robots = int(n_robots)
+        if n_robots <= 0:
+            raise ValueError(f"n_robots must be positive, got {n_robots}")
+        self._h = C.c_void_p()
+        self.cfg, self.n_robots = cfg, n_robots
+        _check(lib().kc_fleet_create(C.byref(cfg), C.byref(follower) if follower is not None else None,
+                                     n_robots, C.byref(self._h)))
+        self.planner = Planner._borrow(C.c_void_p(lib().kc_fleet_planner(self._h)), cfg)
+        self._res = (FleetResult * n_robots)()
+        self._info = (DwaInfo * n_robots)()
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            lib().kc_fleet_destroy(self._h)
+            self._h = C.c_void_p()
+            self.planner._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _robot(self, r):
+        r = int(r)
+        if not 0 <= r < self.n_robots:
+            raise IndexError(f"robot {r} out of range [0, {self.n_robots})")
+        return r
+
+    def set_current_path(self, r, points, interpolate=True):
+        r = self._robot(r)
+        pts = np.asarray(points, dtype=np.float32)
+        x, y = _f32(pts[:, 0]), _f32(pts[:, 1])
+        _check(lib().kc_fleet_set_current_path(self._h, r, _fp(x), _fp(y), len(x), 1 if interpolate else 0))
+
+    def clear_current_path(self, r):
+        _check(lib().kc_fleet_clear_current_path(self._h, self._robot(r)))
+
+    def set_current_states(self, states):
+        """states: [R x 4] (x, y, yaw, speed) or [R x 3] (speed 0)."""
+        st = np.asarray(states, dtype=np.float64)
+        if st.ndim == 2 and st.shape == (self.n_robots, 3):
+            st = np.concatenate([st, np.zeros((self.n_robots, 1))], axis=1)
+        st = _fleet_rows(st, self.n_robots, 4, "states")
+        _check(lib().kc_fleet_set_current_states(self._h, _dp(st)))
+
+    def set_control_limits(self, vx_max, vy_max, omega_max):
+        _check(lib().kc_fleet_set_control_limits(self._h, C.c_double(vx_max), C.c_double(vy_max),
+                                                 C.c_double(omega_max)))
+
+    def compute_velocity_commands(self, vels, clouds=None, scans=None):
+        """One step of every robot. vels: [R x 3]; clouds (list of [n_r x 3] arrays, or (xyz, offsets,
+        counts)) or scans (list of (ranges, angles), or (ranges, angles, offsets, counts)). Returns a
+        dict of numpy arrays [R]: found, cost, slot, n_points, n_slots, n_admissible, cmd [R x 3], and
+        info (record array of the DwaInfo fields)."""
+        R = self.n_robots
+        v = _fleet_rows(vels, R, 3, "vels")
+        if (clouds is None) == (scans is None):
+            raise ValueError("pass exactly one of clouds= or scans=")
+        if clouds is not None:
+            xyz, off, cnt = fleet_pack_clouds(R, clouds)
+            rc = lib().kc_fleet_compute_cloud(self._h, _dp(v), _fp(xyz), off.ctypes.data_as(C.POINTER(C.c_int64)),
+                                              cnt.ctypes.data_as(C.POINTER(C.c_int32)), self._res, self._info)
+        else:
+            rr, aa, off, cnt = fleet_pack_scans(R, scans)
+            rc = lib().kc_fleet_compute_scan(self._h, _dp(v), _dp(rr), _dp(aa),
+                                             off.ctypes.data_as(C.POINTER(C.c_int64)),
+                                             cnt.ctypes.data_as(C.POINTER(C.c_int32)), self._res, self._info)
+        _check(rc)
+        res = np.ctypeslib.as_array(self._res).copy()
+        out = {k: res[k].copy() for k in ("found", "cost", "slot", "n_points", "n_slots", "n_admissible")}
+        out["found"] = out["found"].astype(bool)
+        out["cmd"] = res["cmd"].copy()
+        out["info"] = np.ctypeslib.as_array(self._info).copy().view(np.recarray)
+        return out
+
+    def get_trajectory(self, r):
+        """The winner of robot r's last step, as DWA.compute_velocity_commands returns it."""
+        res = CycleResult()
+        _check(lib().kc_fleet_get_trajectory(self._h, self._robot(r), C.byref(res)))
+        return TrajSearchResult(res)
+
+    def is_goal_reached(self):
+        out = np.zeros(self.n_robots, np.int32)
+        _check(lib().kc_fleet_is_goal_reached(self._h, out.ctypes.data_as(C.POINTER(C.c_int32))))
+        return out.astype(bool)
 
 
 class CollisionChecker:

@@ -99,6 +99,39 @@ int32_t ensure_device();  // selects the device (LOCAL_RANK aware) once per proc
 int sm_count();
 int device_index();  // the CUDA device this process's handles live on
 
+// ---- batched launch set of independent robots (kc_planner.cu) --------------------------------
+// Used by kc_planner_batch_cloud (every robot on the planner's own path and horizon) and by the
+// fleet controller (kc_dwa.cu: every robot with its own path, horizon, tracked segment and sensor).
+
+// TrajectorySampler::updateHorizon (trajectory_sampler.cpp:316-326): clamps `horizon` to
+// [2 time_step, base_horizon] in place and returns the points per trajectory it gives.
+int32_t horizon_points(double time_step, double base_horizon, double &horizon);
+
+struct BatchPath {  // a robot's reference path: host X / Y (segment length and step), device X / Y / acc
+  const float *hX = nullptr, *hY = nullptr;
+  const float *dX = nullptr, *dY = nullptr, *dAcc = nullptr;
+  int32_t n = 0;
+  float total_length = 0.0f;
+};
+struct BatchRobot {
+  const double *vel = nullptr, *pose = nullptr;  // [3] each
+  int32_t P = 0;                                 // points per trajectory (<= the planner's base horizon)
+  BatchPath path;
+  int32_t seg_start = 0, seg_count = 0;  // tracked segment (Path::getPart range)
+  int64_t offset = 0;                    // sensor slice: `count` points / beams from `offset`
+  int32_t count = 0;
+};
+struct BatchSensor {  // one sensor kind for every robot of a call
+  bool cloud = true;
+  const float *xyz = nullptr;                      // clouds: [n x 3], world frame
+  const double *ranges = nullptr, *angles = nullptr;  // scans: beam arrays
+};
+// One control cycle for R robots, chunk after chunk of launch sets. results [R] always; cycles [R]
+// (may be NULL) also receives every robot's winner record (rows point into the planner's host
+// copy, valid until its next call).
+int32_t planner_batch(kc_planner *p, int32_t R, const BatchRobot *robots, const BatchSensor &sensor,
+                      kc_batch_result *results, kc_cycle_result *cycles);
+
 #ifdef __CUDACC__
 // ---- warp helpers ----------------------------------------------------------------------------
 constexpr unsigned FULL = 0xffffffffu;

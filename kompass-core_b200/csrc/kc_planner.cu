@@ -188,7 +188,12 @@ struct kc_planner {
   std::vector<RobotCtx> batch_ctx;
   std::vector<int> batch_starts;  // chunk boundaries of the resident batch (last entry = batch_R)
   int32_t batch_chunk_max = kBatchChunkDefault;  // tuning key 12: robots per launch set of a sweep (<= kBatchChunk)
+  std::vector<int32_t> batch_chunk_P, batch_chunk_S;  // per chunk: largest P and tracked segment (launch geometry)
+  int32_t batch_P = 0;        // largest P of the batch: stride of its result records
+  bool batch_general = false;  // the batch's ctxs take the tilted-sensor rollout (scans through a tilted mount)
   DevBuf<float> d_batch_xyz;
+  DevBuf<double> d_batch_scan;     // scans: per robot ranges | angles, in robot order
+  PinnedBuf<double> h_batch_scan;  // their page-locked staging
   DevBuf<uint8_t> d_batch_stage;
   size_t batch_zero_words = 0, batch_sph_words = 0;
   int32_t batch_max_sensor = 0, batch_max_slots = 0, batch_max_qcells = 0, batch_dil_words = 0;
@@ -434,10 +439,24 @@ int32_t fill_collision_window(const kc_planner_config &c, double x_lo, double x_
   return KC_OK;
 }
 
+// the planner's own reference path (kc_planner_set_path), as the single-robot entry points use it
+BatchPath own_path(const kc_planner *p) {
+  BatchPath b;
+  b.hX = p->hX.data();
+  b.hY = p->hY.data();
+  b.dX = p->d_path.ptr;
+  b.dY = p->d_path.ptr + p->path_n;
+  b.dAcc = p->d_path.ptr + 2 * (size_t)p->path_n;
+  b.n = p->path_n;
+  b.total_length = p->path_len;
+  return b;
+}
+
 // Fill everything of the ctx that does not depend on device pointers. Returns KC_OK or an error.
-int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3],
-                         const SensorDesc &sd, int32_t seg_start, int32_t seg_count, bool want_coll,
-                         bool want_cost, float D, const double cost_pose[3], const Axes &ax,
+// P: points per trajectory of this robot; path: its reference path.
+int32_t fill_ctx_scalars(kc_planner *p, int32_t P, const BatchPath &path, const double vel[3],
+                         const double pose[3], const SensorDesc &sd, int32_t seg_start, int32_t seg_count,
+                         bool want_coll, bool want_cost, float D, const double cost_pose[3], const Axes &ax,
                          RobotCtx &cx, Sizes &sz) {
   const kc_planner_config &c = p->cfg;
   memset(&cx, 0, sizeof(cx));
@@ -445,7 +464,7 @@ int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3
   cx.pose_y = pose[1];
   cx.pose_yaw = pose[2];
   cx.dt = (double)(float)c.time_step;
-  cx.P = p->P;
+  cx.P = P;
   cx.n_slots = ax.n_slots;
   cx.n_rows = (int32_t)ax.vx.size();
   cx.nvy = ax.nvy;
@@ -457,7 +476,7 @@ int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3
   sz.n_sensor = sd.n;
   sz.n_slots = ax.n_slots;
 
-  const double reach = ax.max_speed * (double)(p->P - 1) * cx.dt * 1.001 + 1e-3;
+  const double reach = ax.max_speed * (double)(P - 1) * cx.dt * 1.001 + 1e-3;
 
   // ---- collision world (ref: collision_check.h:91-136, collision_check.cpp:125-135) ----
   cx.coll_enabled = (want_coll && sd.n > 0) ? 1 : 0;
@@ -506,32 +525,32 @@ int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3
   cx.acc1 = (float)c.vy_acc;
   cx.acc2 = (float)c.omega_acc;
   cx.obs_enabled = (want_cost && sd.n > 0 && c.w_obstacles > 0.0) ? 1 : 0;
-  cx.path_enabled = (want_cost && p->path_len > 0.0f) ? 1 : 0;
-  cx.path_n = p->path_n;
-  cx.path_len = p->path_len;
+  cx.path_enabled = (want_cost && path.total_length > 0.0f) ? 1 : 0;
+  cx.path_n = path.n;
+  cx.path_len = path.total_length;
   cx.seg_start = 0;
   cx.seg_count = 0;
   if (want_cost) {
     // ref: path.cpp:80-86 Path::getPart range check
-    KC_REQUIRE(seg_start >= 0 && seg_count >= 1 && seg_start + seg_count <= p->path_n,
+    KC_REQUIRE(seg_start >= 0 && seg_count >= 1 && seg_start + seg_count <= path.n,
                KC_ERR_OUT_OF_RANGE,
                "Invalid range for path part. Maximum path size is %d, but requested part start= "
                "%d, and requested end= %d",
-               p->path_n, seg_start, seg_start + seg_count - 1);
+               path.n, seg_start, seg_start + seg_count - 1);
     cx.seg_start = seg_start;
     cx.seg_count = seg_count;
     // ref: path.h:85-91 View::totalSegmentLength (float sum of float norms, index order)
     float len = 0.0f;
     for (int i = 0; i + 1 < seg_count; ++i) {
-      const float ddx = p->hX[seg_start + i] - p->hX[seg_start + i + 1];
-      const float ddy = p->hY[seg_start + i] - p->hY[seg_start + i + 1];
+      const float ddx = path.hX[seg_start + i] - path.hX[seg_start + i + 1];
+      const float ddy = path.hY[seg_start + i] - path.hY[seg_start + i + 1];
       len += std::sqrt(ddx * ddx + (ddy * ddy + 0.0f));
     }
     cx.seg_len = len;
     double step = 0.0;
     for (int i = 0; i + 1 < seg_count; ++i)
-      step = std::max(step, std::hypot((double)p->hX[seg_start + i] - (double)p->hX[seg_start + i + 1],
-                                       (double)p->hY[seg_start + i] - (double)p->hY[seg_start + i + 1]));
+      step = std::max(step, std::hypot((double)path.hX[seg_start + i] - (double)path.hX[seg_start + i + 1],
+                                       (double)path.hY[seg_start + i] - (double)path.hY[seg_start + i + 1]));
     cx.seg_step = (float)(step * (1.0 + 1e-6) + 1e-9);
     if (!(cx.seg_step < 1e30f)) cx.seg_step = 1e30f;  // non-finite path: disables the pruning
   }
@@ -539,7 +558,7 @@ int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3
   // analytic reach set of this cycle's velocity window (see cell_reachable); non-holonomic only
   cx.reach_mask = 0;
   if (p->use_reach_mask && want_coll && want_cost && c.control_type != KC_OMNI && ax.n_slots > 0 &&
-      p->P >= 4 && !ax.vx.empty() && !ax.om.empty()) {
+      P >= 4 && !ax.vx.empty() && !ax.om.empty()) {
     double vf = 0.0, vr = 0.0, om_lo = ax.om.front(), om_hi = ax.om.front();
     for (double v : ax.vx) {
       vf = std::max(vf, v);
@@ -549,7 +568,7 @@ int32_t fill_ctx_scalars(kc_planner *p, const double vel[3], const double pose[3
       om_lo = std::min(om_lo, o);
       om_hi = std::max(om_hi, o);
     }
-    const int n = p->P - 2;
+    const int n = P - 2;
     cx.reach_mask = 1;
     cx.rm_n = n;
     cx.rm_px = (float)pose[0];
@@ -641,9 +660,10 @@ int32_t reserve_workspace(kc_planner *p, int R, size_t zero_words, size_t sph_wo
 }
 
 // r: workspace slot of this robot; r_result: slot of its result record (the batch reuses the
-// workspace chunk after chunk but keeps one result record per robot)
-void bind_workspace(kc_planner *p, RobotCtx &cx, int r, size_t zero_words, size_t bitmap_words,
-                    size_t sph_words, int32_t max_sensor, int32_t max_slots, int32_t P,
+// workspace chunk after chunk but keeps one result record per robot). P: the launch set's largest
+// points per trajectory, which sizes the per-robot strides (a robot's own cx.P may be smaller).
+void bind_workspace(kc_planner *p, RobotCtx &cx, const BatchPath &path, int r, size_t zero_words,
+                    size_t bitmap_words, size_t sph_words, int32_t max_sensor, int32_t max_slots, int32_t P,
                     int r_result = -1) {
   uint32_t *z = p->d_zero.ptr + (size_t)r * zero_words;
   {
@@ -714,9 +734,9 @@ void bind_workspace(kc_planner *p, RobotCtx &cx, int r, size_t zero_words, size_
   uint8_t *rb = p->d_result.ptr + (size_t)(r_result >= 0 ? r_result : r) * res_bytes;
   cx.result = reinterpret_cast<ResultHeader *>(rb);
   cx.res_rows = reinterpret_cast<float *>(rb + sizeof(ResultHeader));
-  cx.pathX = p->d_path.ptr;
-  cx.pathY = p->d_path.ptr + p->path_n;
-  cx.pathAcc = p->d_path.ptr + 2 * (size_t)p->path_n;
+  cx.pathX = path.dX;
+  cx.pathY = path.dY;
+  cx.pathAcc = path.dAcc;
 }
 
 int pick_eval_warps(int P, int S, int dil_words, size_t &smem) {  // k_eval_rows
@@ -1094,14 +1114,15 @@ int32_t run_single(kc_planner *p, const double vel[3], const double pose[3], con
   Sizes sz;
   const float D = p->cfg.max_local_range / 3.0f;  // ref: cost_evaluator.h:179 via dwa.h:223
   p->general_bound = false;
-  KC_TRY(fill_ctx_scalars(p, vel, pose, sd, seg_start, seg_count, true, mode == 0, D, pose, ax, cx, sz));
+  KC_TRY(fill_ctx_scalars(p, p->P, own_path(p), vel, pose, sd, seg_start, seg_count, true, mode == 0, D, pose,
+                          ax, cx, sz));
   p->general_bound = cx.coll_general != 0;  // tilted mount + scan: the oriented-cube rollout kernel
   const double reach = ax.max_speed * (double)(p->P - 1) * cx.dt * 1.001 + 1e-3;
   set_grid_window(cx, (float)pose[0], (float)pose[1], reach + (double)D * 1.001 + 1e-3, reach + 1e-3);
 
   const size_t zw = zero_words_per_robot(sz.bitmap_words);
   KC_TRY(reserve_workspace(p, 1, zw, sz.sph_words, sd.n, ax.n_slots, p->P));
-  bind_workspace(p, cx, 0, zw, sz.bitmap_words, sz.sph_words, sd.n, ax.n_slots, p->P);
+  bind_workspace(p, cx, own_path(p), 0, zw, sz.bitmap_words, sz.sph_words, sd.n, ax.n_slots, p->P);
   const int32_t dil_words = plan_dilation(cx, sz.bitmap_words);
   if (mode == 1) {
     const size_t nv = (size_t)ax.n_slots * (p->P - 1);
@@ -1503,6 +1524,8 @@ void kc_planner_destroy(kc_planner *p) {
   p->h_adm.release();
   p->d_bank.release();
   p->d_batch_xyz.release();
+  p->d_batch_scan.release();
+  p->h_batch_scan.release();
   p->d_batch_stage.release();
   for (kc_planner::GraphSlot &g : p->graphs)
     if (g.exec) cudaGraphExecDestroy(g.exec);
@@ -1567,11 +1590,8 @@ int32_t kc_planner_num_slots_last(const kc_planner *p) { return p ? p->last_slot
 int32_t kc_planner_set_prediction_horizon(kc_planner *p, double horizon, int32_t *n_points) {
   KC_REQUIRE(p, KC_ERR_INVALID_ARG, "null handle");
   KC_TRY(kc::ensure_device());
-  const double min_h = 2.0 * p->cfg.time_step;  // trajectory_sampler.cpp:316-326
-  if (horizon < min_h) horizon = min_h;
-  if (horizon > p->base_horizon) horizon = p->base_horizon;
+  p->P = horizon_points(p->cfg.time_step, p->base_horizon, horizon);
   p->horizon = horizon;
-  p->P = (int32_t)(size_t)(horizon / p->cfg.time_step);
   if (n_points) *n_points = p->P;
   return KC_OK;
 }
@@ -1763,7 +1783,7 @@ int32_t kc_cost_evaluate(kc_planner *p, int32_t n_traj, int32_t P, const float *
   RobotCtx cx;
   Sizes sz;
   const double zero3[3] = {0, 0, 0};
-  KC_TRY(fill_ctx_scalars(p, zero3, zero3, sd, seg_start, seg_count, false, true, p->cost_D,
+  KC_TRY(fill_ctx_scalars(p, p->P, own_path(p), zero3, zero3, sd, seg_start, seg_count, false, true, p->cost_D,
                           p->cost_pose, ax, cx, sz));
   cx.n_traj = n_traj;
   cx.in_vx = dvx;
@@ -1797,7 +1817,7 @@ int32_t kc_cost_evaluate(kc_planner *p, int32_t n_traj, int32_t P, const float *
   }
   const size_t zw = zero_words_per_robot(0);
   KC_TRY(reserve_workspace(p, 1, zw, 0, sd.n, n_traj, P));
-  bind_workspace(p, cx, 0, zw, 0, 0, sd.n, n_traj, P);
+  bind_workspace(p, cx, own_path(p), 0, zw, 0, 0, sd.n, n_traj, P);
   SensorDesc sdl = sd;
   const StageLayout L = plan_stage(ax, sdl);
   KC_TRY(p->h_stage.reserve(L.total));
@@ -1902,7 +1922,8 @@ int32_t kc_planner_replay(kc_planner *p, int32_t first_slot, int32_t n_cycles, c
     sd.is_cloud = 1;
     sd.n = p->bank_counts[s];
     Sizes sz;
-    KC_TRY(fill_ctx_scalars(p, vel, pose, sd, seg_start, seg_count, true, true, D, pose, ax, ctxs[s], sz));
+    KC_TRY(fill_ctx_scalars(p, p->P, own_path(p), vel, pose, sd, seg_start, seg_count, true, true, D, pose, ax,
+                            ctxs[s], sz));
     const double reach = ax.max_speed * (double)(p->P - 1) * ctxs[s].dt * 1.001 + 1e-3;
     set_grid_window(ctxs[s], (float)pose[0], (float)pose[1], reach + (double)D * 1.001 + 1e-3, reach + 1e-3);
     szmax.bitmap_words = std::max(szmax.bitmap_words, sz.bitmap_words);
@@ -1924,7 +1945,7 @@ int32_t kc_planner_replay(kc_planner *p, int32_t first_slot, int32_t n_cycles, c
   int32_t dil_words = 0;
   for (int s = 0; s < ns; ++s) {
     RobotCtx &cx = ctxs[s];
-    bind_workspace(p, cx, 0, zw, szmax.bitmap_words, szmax.sph_words, max_sensor, ax.n_slots, p->P);
+    bind_workspace(p, cx, own_path(p), 0, zw, szmax.bitmap_words, szmax.sph_words, max_sensor, ax.n_slots, p->P);
     dil_words = std::max(dil_words, plan_dilation(cx, (size_t)cx.bm_rows * cx.bm_wpr));
     cx.ax_vx = reinterpret_cast<const double *>(ds + L.vx_off + shift);
     cx.ax_vy = reinterpret_cast<const double *>(ds + L.vy_off + shift);
@@ -2225,81 +2246,130 @@ int32_t kc_planner_bruteforce_obstacle_costs(kc_planner *p, float *costs, float 
   return KC_OK;
 }
 
+}  // extern "C"
+
 // ---- batched multi-robot sweep ---------------------------------------------------------------
 // The sweep runs chunk after chunk of kBatchChunk robots: one launch set per chunk (blockIdx.y =
 // robot within the chunk) on a workspace sized for one chunk, so device memory stays bounded
-// (~18 MB per robot of the chunk instead of per robot of the sweep) and the clouds of chunk k+1 are
-// uploaded while chunk k computes.
+// (~18 MB per robot of the chunk instead of per robot of the sweep) and the sensor data of chunk k+1
+// is uploaded while chunk k computes.
+//
+// Robots of one launch set may differ in points per trajectory (P: a horizon shortened on path
+// curvature), tracked segment length (S: near the path end), velocity slots and sensor count. Every
+// kernel takes these bounds from its robot's ctx; the launch geometry takes the chunk's largest P and
+// S only to size the per-warp shared-memory carve-outs and the warp count, which a smaller robot
+// then fills in part. The per-robot strides of the workspace (heading table, trajectory rows,
+// result record) are set by the largest P of the whole batch.
 
-static int32_t batch_launch_chunk(kc_planner *p, int ci) {
+namespace {
+
+int32_t batch_launch_chunk(kc_planner *p, int ci) {
   const int c0 = p->batch_starts[ci], Rc = p->batch_starts[ci + 1] - c0;
   const RobotCtx *d_ctx = reinterpret_cast<const RobotCtx *>(p->d_batch_stage.ptr) + c0;
   return launch_cycle(p, d_ctx, Rc, p->batch_zero_words * (size_t)Rc, p->batch_sph_words * (size_t)Rc,
-                      p->batch_max_sensor, p->batch_max_slots, p->P, p->batch_ctx[0].seg_count,
+                      p->batch_max_sensor, p->batch_max_slots, p->batch_chunk_P[ci], p->batch_chunk_S[ci],
                       p->batch_max_sensor > 0, 0, nullptr, nullptr, p->batch_max_qcells,
                       p->batch_dil_words);
 }
 
-static int32_t batch_launch(kc_planner *p) {
+int32_t batch_launch(kc_planner *p) {
   for (size_t ci = 0; ci + 1 < p->batch_starts.size(); ++ci) KC_TRY(batch_launch_chunk(p, (int)ci));
   return KC_OK;
 }
 
-static int32_t batch_fetch(kc_planner *p, kc_batch_result *results) {
+// results [R]; cycles [R] or NULL: with cycles the whole records (header | rows) come back in one
+// copy, without them only the R headers (strided gather)
+int32_t batch_fetch(kc_planner *p, kc_batch_result *results, kc_cycle_result *cycles) {
   const int R = p->batch_R;
-  const size_t res_bytes = align_up(sizeof(ResultHeader) + sizeof(float) * (5 * (size_t)p->P));
-  // strided gather of the R result headers: the only data that leaves the device
-  KC_CUDA(cudaMemcpy2DAsync(p->h_result.ptr, sizeof(ResultHeader), p->d_result.ptr, res_bytes,
-                            sizeof(ResultHeader), R, cudaMemcpyDeviceToHost, p->stream));
+  const size_t res_bytes = align_up(sizeof(ResultHeader) + sizeof(float) * (5 * (size_t)p->batch_P));
+  const size_t hstride = cycles ? res_bytes : sizeof(ResultHeader);
+  if (cycles)
+    KC_CUDA(cudaMemcpyAsync(p->h_result.ptr, p->d_result.ptr, (size_t)R * res_bytes, cudaMemcpyDeviceToHost,
+                            p->stream));
+  else  // strided gather of the R result headers: the only data that leaves the device
+    KC_CUDA(cudaMemcpy2DAsync(p->h_result.ptr, sizeof(ResultHeader), p->d_result.ptr, res_bytes,
+                              sizeof(ResultHeader), R, cudaMemcpyDeviceToHost, p->stream));
   KC_CUDA(cudaStreamSynchronize(p->stream));
-  const ResultHeader *h = reinterpret_cast<const ResultHeader *>(p->h_result.ptr);
   p->heavy_seen = false;
   for (int r = 0; r < R; ++r) {
-    if (h[r].heavy_cells) p->heavy_seen = true;  // feedback for the next sweep's launch set
-    results[r].found = h[r].n_admissible ? h[r].found : 0;
-    results[r].cost = h[r].n_admissible ? h[r].cost : 0.0f;
-    results[r].slot = h[r].slot;
-    results[r].n_admissible = h[r].n_admissible;
-    results[r].n_slots = p->batch_ctx[r].n_slots;
+    uint8_t *rec = p->h_result.ptr + (size_t)r * hstride;
+    const RobotCtx &cx = p->batch_ctx[r];
+    // a robot without velocity slots has no launch work: its record is what a single cycle reports
+    if (cycles && cx.n_slots == 0) memset(rec, 0, sizeof(ResultHeader) + sizeof(float) * 5 * (size_t)cx.P);
+    const ResultHeader &h = *reinterpret_cast<const ResultHeader *>(rec);
+    if (h.heavy_cells) p->heavy_seen = true;  // feedback for the next sweep's launch set
+    results[r].found = h.n_admissible ? h.found : 0;
+    results[r].cost = h.n_admissible ? h.cost : 0.0f;
+    results[r].slot = h.slot;
+    results[r].n_admissible = h.n_admissible;
+    results[r].n_slots = cx.n_slots;
+    if (cycles) {
+      const bool heavy = p->heavy_seen;
+      fill_result(p, rec, cx.P, cx.n_slots, &cycles[r]);
+      p->heavy_seen = heavy;
+    }
   }
   return KC_OK;
 }
 
-int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, const double *pose,
-                               const float *xyz, const int64_t *offsets, const int32_t *counts,
-                               int32_t seg_start, int32_t seg_count, kc_batch_result *results) {
-  KC_REQUIRE(p && vel && pose && offsets && counts && results, KC_ERR_INVALID_ARG, "null argument");
+}  // namespace
+
+namespace kc {
+
+int32_t horizon_points(double time_step, double base_horizon, double &horizon) {
+  const double min_h = 2.0 * time_step;  // trajectory_sampler.cpp:316-326
+  if (horizon < min_h) horizon = min_h;
+  if (horizon > base_horizon) horizon = base_horizon;
+  return (int32_t)(size_t)(horizon / time_step);
+}
+
+int32_t planner_batch(kc_planner *p, int32_t R, const BatchRobot *rb, const BatchSensor &sen,
+                      kc_batch_result *results, kc_cycle_result *cycles) {
+  KC_REQUIRE(p && rb && results, KC_ERR_INVALID_ARG, "null argument");
   KC_REQUIRE(R > 0, KC_ERR_INVALID_ARG, "n_robots must be positive");
-  KC_REQUIRE(p->path_n >= 2, KC_ERR_INVALID_ARG, "reference path not set");
   KC_TRY(kc::ensure_device());
   const bool timing = getenv("KC_BATCH_TIMING") != nullptr;  // developer: host-side split on stderr
   const auto t_begin = std::chrono::steady_clock::now();
   auto since = [&] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_begin).count(); };
   p->heavy_bound = p->batch_heavy = p->heavy_kernel_on();
-  p->general_bound = false;  // clouds are world-frame data: identity octree frame
   const float D = p->cfg.max_local_range / 3.0f;
   std::vector<Axes> axes(R);
   p->batch_ctx.assign(R, RobotCtx());
   Sizes szmax;
-  int32_t max_sensor = 0, max_slots = 0;
-  int64_t total_pts = 0;
+  int32_t max_sensor = 0, max_slots = 0, Pmax = 0;
+  int64_t total_pts = 0, scan_total = 0;
   for (int r = 0; r < R; ++r) {
-    KC_REQUIRE(counts[r] >= 0 && offsets[r] >= 0, KC_ERR_INVALID_ARG, "bad cloud extents");
-    total_pts = std::max<int64_t>(total_pts, offsets[r] + counts[r]);
+    KC_REQUIRE(rb[r].count >= 0 && rb[r].offset >= 0, KC_ERR_INVALID_ARG, "robot %d: bad sensor extents", r);
+    KC_REQUIRE(rb[r].vel && rb[r].pose, KC_ERR_INVALID_ARG, "robot %d: null velocity or pose", r);
+    KC_REQUIRE(rb[r].P >= 2, KC_ERR_INVALID_ARG, "robot %d: %d points per trajectory", r, rb[r].P);
+    KC_REQUIRE(rb[r].path.n >= 2 && rb[r].path.hX && rb[r].path.hY && rb[r].path.dX, KC_ERR_INVALID_ARG,
+               "robot %d: reference path not set", r);
+    total_pts = std::max<int64_t>(total_pts, rb[r].offset + rb[r].count);
+    scan_total += 2 * (int64_t)rb[r].count;
+    Pmax = std::max(Pmax, rb[r].P);
   }
-  KC_REQUIRE(total_pts == 0 || xyz, KC_ERR_INVALID_ARG, "null cloud");
+  if (sen.cloud)
+    KC_REQUIRE(total_pts == 0 || sen.xyz, KC_ERR_INVALID_ARG, "null cloud");
+  else
+    KC_REQUIRE(total_pts == 0 || (sen.ranges && sen.angles), KC_ERR_INVALID_ARG, "null scan arrays");
   size_t axes_bytes = 0;
+  bool general = false;
   for (int r = 0; r < R; ++r) {
-    enumerate_axes(p->cfg, vel + 3 * r, axes[r]);
+    const BatchRobot &b = rb[r];
+    enumerate_axes(p->cfg, b.vel, axes[r]);
     SensorDesc sd;
-    sd.is_cloud = 1;
-    sd.n = counts[r];
+    sd.is_cloud = sen.cloud ? 1 : 0;
+    sd.n = b.count;
     Sizes sz;
-    KC_TRY(fill_ctx_scalars(p, vel + 3 * r, pose + 3 * r, sd, seg_start, seg_count, true, true, D,
-                            pose + 3 * r, axes[r], p->batch_ctx[r], sz));
-    const double reach = axes[r].max_speed * (double)(p->P - 1) * p->batch_ctx[r].dt * 1.001 + 1e-3;
-    set_grid_window(p->batch_ctx[r], (float)pose[3 * r], (float)pose[3 * r + 1],
-                    reach + (double)D * 1.001 + 1e-3, reach + 1e-3);
+    RobotCtx &cx = p->batch_ctx[r];
+    KC_TRY(fill_ctx_scalars(p, b.P, b.path, b.vel, b.pose, sd, b.seg_start, b.seg_count, true, true, D, b.pose,
+                            axes[r], cx, sz));
+    // clouds arrive in the world frame (identity octree frame); a scan's frame follows its robot's pose
+    // through the shared mount, so whether it is tilted is the same for every robot
+    if (r == 0) general = cx.coll_general != 0;
+    KC_REQUIRE((cx.coll_general != 0) == general, KC_ERR_UNSUPPORTED, "mixed sensor frames in one batch");
+    const double reach = axes[r].max_speed * (double)(b.P - 1) * cx.dt * 1.001 + 1e-3;
+    set_grid_window(cx, (float)b.pose[0], (float)b.pose[1], reach + (double)D * 1.001 + 1e-3, reach + 1e-3);
     szmax.bitmap_words = std::max(szmax.bitmap_words, sz.bitmap_words);
     szmax.sph_words = std::max(szmax.sph_words, sz.sph_words);
     max_sensor = std::max(max_sensor, sd.n);
@@ -2307,6 +2377,7 @@ int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, cons
     axes_bytes += align_up((axes[r].vx.size() + axes[r].vy.size() + axes[r].om.size()) * 8 +
                            axes[r].row_off.size() * 4 + 64);
   }
+  p->general_bound = p->batch_general = general;
   const size_t zw = zero_words_per_robot(szmax.bitmap_words);
   const int C = std::min(R, std::max(1, std::min(p->batch_chunk_max, kBatchChunk)));
   // chunk boundaries: the first chunk's clouds cannot be uploaded behind any computation, so the sweep
@@ -2315,16 +2386,31 @@ int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, cons
   p->batch_starts.clear();
   for (int c0 = 0, step = std::min(8, C); c0 < R; c0 += step, step = std::min(2 * step, C)) p->batch_starts.push_back(c0);
   p->batch_starts.push_back(R);
+  const size_t n_chunks = p->batch_starts.size() - 1;
+  p->batch_chunk_P.assign(n_chunks, 0);
+  p->batch_chunk_S.assign(n_chunks, 0);
   std::vector<int> slot_of(R);
-  for (size_t c = 0; c + 1 < p->batch_starts.size(); ++c)
-    for (int r = p->batch_starts[c]; r < p->batch_starts[c + 1]; ++r) slot_of[r] = r - p->batch_starts[c];
-  KC_TRY(reserve_workspace(p, C, zw, szmax.sph_words, max_sensor, max_slots, p->P));
+  for (size_t c = 0; c < n_chunks; ++c)
+    for (int r = p->batch_starts[c]; r < p->batch_starts[c + 1]; ++r) {
+      slot_of[r] = r - p->batch_starts[c];
+      p->batch_chunk_P[c] = std::max(p->batch_chunk_P[c], rb[r].P);
+      p->batch_chunk_S[c] = std::max(p->batch_chunk_S[c], p->batch_ctx[r].seg_count);
+    }
+  KC_TRY(reserve_workspace(p, C, zw, szmax.sph_words, max_sensor, max_slots, Pmax));
   {
-    const size_t res_bytes = align_up(sizeof(ResultHeader) + sizeof(float) * (5 * (size_t)p->P));
+    const size_t res_bytes = align_up(sizeof(ResultHeader) + sizeof(float) * (5 * (size_t)Pmax));
     KC_TRY(p->d_result.reserve((size_t)R * res_bytes));
     KC_TRY(p->h_result.reserve((size_t)R * res_bytes));
   }
-  KC_TRY(p->d_batch_xyz.reserve((size_t)std::max<int64_t>(total_pts, 1) * 3));
+  std::vector<int64_t> scan_off;
+  if (sen.cloud) {
+    KC_TRY(p->d_batch_xyz.reserve((size_t)std::max<int64_t>(total_pts, 1) * 3));
+  } else {
+    KC_TRY(p->d_batch_scan.reserve((size_t)std::max<int64_t>(scan_total, 1)));
+    KC_TRY(p->h_batch_scan.reserve((size_t)std::max<int64_t>(scan_total, 1)));
+    scan_off.assign(R + 1, 0);
+    for (int r = 0; r < R; ++r) scan_off[r + 1] = scan_off[r] + 2 * (int64_t)rb[r].count;
+  }
   if (!p->copy) {
     KC_CUDA(cudaStreamCreateWithFlags(&p->copy, cudaStreamNonBlocking));
     KC_CUDA(cudaEventCreateWithFlags(&p->ev_copy, cudaEventDisableTiming));
@@ -2338,7 +2424,8 @@ int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, cons
   for (int r = 0; r < R; ++r) {
     RobotCtx &cx = p->batch_ctx[r];
     const Axes &a = axes[r];
-    bind_workspace(p, cx, slot_of[r], zw, szmax.bitmap_words, szmax.sph_words, max_sensor, max_slots, p->P, r);
+    bind_workspace(p, cx, rb[r].path, slot_of[r], zw, szmax.bitmap_words, szmax.sph_words, max_sensor, max_slots,
+                   Pmax, r);
     if (szmax.bitmap_words <= kDilMaxWords)  // every robot's bitmap must fit the shared smem carve-out
       batch_dil = std::max(batch_dil, plan_dilation(cx, (size_t)cx.bm_rows * cx.bm_wpr));
     cx.ax_vx = reinterpret_cast<const double *>(ds + o);
@@ -2353,12 +2440,16 @@ int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, cons
     cx.row_off = reinterpret_cast<const int32_t *>(ds + o);
     memcpy(hs + o, a.row_off.data(), a.row_off.size() * 4);
     o = align_up(o + a.row_off.size() * 4);
-    cx.sensor = p->d_batch_xyz.ptr + 3 * offsets[r];
+    if (sen.cloud)
+      cx.sensor = p->d_batch_xyz.ptr + 3 * rb[r].offset;
+    else  // k_prep_points reads a scan as ranges [n] then angles [n]
+      cx.sensor = p->d_batch_scan.ptr + scan_off[r];
     memcpy(hs + sizeof(RobotCtx) * (size_t)r, &cx, sizeof(cx));
   }
   KC_CUDA(cudaMemcpyAsync(ds, hs, o, cudaMemcpyHostToDevice, p->stream));
   p->batch_R = R;
   p->batch_chunk = C;
+  p->batch_P = Pmax;
   p->batch_zero_words = zw;
   p->batch_sph_words = szmax.sph_words;
   p->batch_max_sensor = max_sensor;
@@ -2366,42 +2457,84 @@ int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, cons
   p->batch_dil_words = batch_dil;
   p->batch_max_qcells = 0;
   for (int r = 0; r < R; ++r) p->batch_max_qcells = std::max(p->batch_max_qcells, qcells(p->batch_ctx[r]));
-  // chunk pipeline: the copy stream uploads the point range chunk k needs (a page-locked caller
-  // buffer is DMA-ed directly; pageable memory is staged by the driver while the GPU works on the
-  // previous chunk), the compute stream waits for it and runs chunk k
+  // chunk pipeline: the copy stream uploads the sensor data chunk k needs (a page-locked caller cloud
+  // is DMA-ed directly; pageable memory is staged by the driver, scans through the handle's page-locked
+  // buffer, while the GPU works on the previous chunk), the compute stream waits for it and runs chunk k
   const double t_prep = since();
   int64_t up_lo = 0, up_hi = 0;  // point range already uploaded
-  for (size_t ci = 0; ci + 1 < p->batch_starts.size(); ++ci) {
+  for (size_t ci = 0; ci < n_chunks; ++ci) {
     const int c0 = p->batch_starts[ci], c1 = p->batch_starts[ci + 1];
-    int64_t lo = INT64_MAX, hi = 0;
-    for (int r = c0; r < c1; ++r) {
-      if (counts[r] == 0) continue;
-      lo = std::min<int64_t>(lo, offsets[r]);
-      hi = std::max<int64_t>(hi, offsets[r] + counts[r]);
-    }
-    if (lo < hi && !(lo >= up_lo && hi <= up_hi)) {
-      int64_t a = lo, b = hi;
-      if (up_lo < up_hi && lo >= up_lo && lo <= up_hi) {  // extends the uploaded range upwards
-        a = up_hi;
-        up_hi = hi;
-      } else {  // disjoint layout: restart the bookkeeping with this range
-        up_lo = lo;
-        up_hi = hi;
+    if (sen.cloud) {
+      int64_t lo = INT64_MAX, hi = 0;
+      for (int r = c0; r < c1; ++r) {
+        if (rb[r].count == 0) continue;
+        lo = std::min<int64_t>(lo, rb[r].offset);
+        hi = std::max<int64_t>(hi, rb[r].offset + rb[r].count);
       }
-      if (a < b)
-        KC_CUDA(cudaMemcpyAsync(p->d_batch_xyz.ptr + 3 * a, xyz + 3 * a, (size_t)(b - a) * 12,
-                                cudaMemcpyHostToDevice, p->copy));
+      if (lo < hi && !(lo >= up_lo && hi <= up_hi)) {
+        int64_t a = lo, b = hi;
+        if (up_lo < up_hi && lo >= up_lo && lo <= up_hi) {  // extends the uploaded range upwards
+          a = up_hi;
+          up_hi = hi;
+        } else {  // disjoint layout: restart the bookkeeping with this range
+          up_lo = lo;
+          up_hi = hi;
+        }
+        if (a < b)
+          KC_CUDA(cudaMemcpyAsync(p->d_batch_xyz.ptr + 3 * a, sen.xyz + 3 * a, (size_t)(b - a) * 12,
+                                  cudaMemcpyHostToDevice, p->copy));
+      }
+    } else if (scan_off[c1] > scan_off[c0]) {
+      double *h = p->h_batch_scan.ptr;
+      for (int r = c0; r < c1; ++r) {
+        const size_t n = (size_t)rb[r].count;
+        if (!n) continue;
+        memcpy(h + scan_off[r], sen.ranges + rb[r].offset, n * 8);
+        memcpy(h + scan_off[r] + n, sen.angles + rb[r].offset, n * 8);
+      }
+      KC_CUDA(cudaMemcpyAsync(p->d_batch_scan.ptr + scan_off[c0], h + scan_off[c0],
+                              (size_t)(scan_off[c1] - scan_off[c0]) * 8, cudaMemcpyHostToDevice, p->copy));
     }
     KC_CUDA(cudaEventRecord(p->ev_copy, p->copy));
     KC_CUDA(cudaStreamWaitEvent(p->stream, p->ev_copy, 0));
     KC_TRY(batch_launch_chunk(p, (int)ci));
   }
   const double t_enq = since();
-  const int32_t rc = batch_fetch(p, results);
+  const int32_t rc = batch_fetch(p, results, cycles);
   if (timing)
     fprintf(stderr, "[kc batch] R=%d chunks=%zu host prep %.3f ms, enqueue %.3f ms, wait+fetch %.3f ms\n", R,
-            p->batch_starts.size() - 1, t_prep, t_enq - t_prep, since() - t_enq);
+            n_chunks, t_prep, t_enq - t_prep, since() - t_enq);
   return rc;
+}
+
+}  // namespace kc
+
+extern "C" {
+
+int32_t kc_planner_batch_cloud(kc_planner *p, int32_t R, const double *vel, const double *pose,
+                               const float *xyz, const int64_t *offsets, const int32_t *counts,
+                               int32_t seg_start, int32_t seg_count, kc_batch_result *results) {
+  KC_REQUIRE(p && vel && pose && offsets && counts && results, KC_ERR_INVALID_ARG, "null argument");
+  KC_REQUIRE(R > 0, KC_ERR_INVALID_ARG, "n_robots must be positive");
+  KC_REQUIRE(p->path_n >= 2, KC_ERR_INVALID_ARG, "reference path not set");
+  KC_TRY(kc::ensure_device());
+  std::vector<BatchRobot> rb(R);
+  const BatchPath path = own_path(p);
+  for (int r = 0; r < R; ++r) {
+    KC_REQUIRE(counts[r] >= 0 && offsets[r] >= 0, KC_ERR_INVALID_ARG, "bad cloud extents");
+    rb[r].vel = vel + 3 * r;
+    rb[r].pose = pose + 3 * r;
+    rb[r].P = p->P;
+    rb[r].path = path;
+    rb[r].seg_start = seg_start;
+    rb[r].seg_count = seg_count;
+    rb[r].offset = offsets[r];
+    rb[r].count = counts[r];
+  }
+  BatchSensor sen;
+  sen.cloud = true;
+  sen.xyz = xyz;
+  return planner_batch(p, R, rb.data(), sen, results, nullptr);
 }
 
 int32_t kc_planner_batch_replay(kc_planner *p, int32_t n_iters, float *total_ms,
@@ -2410,7 +2543,7 @@ int32_t kc_planner_batch_replay(kc_planner *p, int32_t n_iters, float *total_ms,
              "no resident batch (call kc_planner_batch_cloud first)");
   KC_TRY(kc::ensure_device());
   p->heavy_bound = p->batch_heavy;  // the resident ctxs were bound with this decision
-  p->general_bound = false;
+  p->general_bound = p->batch_general;
   KC_CUDA(cudaEventRecord(p->ev0, p->stream));
   for (int i = 0; i < n_iters; ++i) KC_TRY(batch_launch(p));
   KC_CUDA(cudaEventRecord(p->ev1, p->stream));
@@ -2418,7 +2551,7 @@ int32_t kc_planner_batch_replay(kc_planner *p, int32_t n_iters, float *total_ms,
   float ms = 0.0f;
   KC_CUDA(cudaEventElapsedTime(&ms, p->ev0, p->ev1));
   if (total_ms) *total_ms = ms;
-  if (results) return batch_fetch(p, results);
+  if (results) return batch_fetch(p, results, nullptr);
   return KC_OK;
 }
 
